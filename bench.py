@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: BERT-large training throughput (sequences/s, whole job) on N B200s.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by the driver as ``python -m torch.distributed.run --nproc-per-node N ...``
 (one rank per GPU, RANK/LOCAL_RANK/WORLD_SIZE/MASTER_* from the env).  Workload = BASELINE.md §2:
@@ -57,6 +57,8 @@ def parse_args():
     ap.add_argument("--virtual-stages", type=int, default=int(os.environ.get("SKY_VIRTUAL_STAGES", "0")))
     ap.add_argument("--slow-rank", type=int, default=-1)
     ap.add_argument("--slowdown", type=float, default=0.0)
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR",
+                    help="write the last timed step's loss and the updated parameters to DIR/*.npy")
     return ap.parse_args()
 
 
@@ -392,6 +394,8 @@ def measure(args, plan, rank, world, local_rank, device):
         last_loss = loss_t.item()
     else:
         launches = int(graph_launches)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, model, last_loss, rank, world, device)
     err = eng.fused.error_code() if eng.fused is not None else 0
     # exposed stage-boundary communication (part of the BASELINE.json metric): per-crossing cost
     # of both fused boundary kernels, measured on ranks 0 / 1 right here, times the crossings a
@@ -452,6 +456,41 @@ def measure(args, plan, rank, world, local_rank, device):
         }
     eng.close()
     return result
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+NPY_HEADER_BYTES = 128
+
+
+def dump_outputs(out_dir, model, loss, rank, world, device):
+    """--dump-outputs: what the timed path produced by its last step, as float32 .npy files: the
+    mean loss (``loss.npy``) and every parameter after that step's SGD update
+    (``param.<global layer index>.<parameter name>.npy``, so the files do not depend on how the
+    layers were split over the GPUs).  A parameter larger than its share of the 64 MB budget is
+    written as a fixed seeded sample of its elements, the same in every run, so that two builds
+    run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+
+    params = []
+    for m in model.model:
+        if m.is_local:
+            first = m.layer_range[0] if m.layer_range else 0
+            for i, layer in enumerate(m.module.layers.children()):
+                params += [(f"param.{first + i:03d}.{n}", p) for n, p in layer.named_parameters()]
+    n_files = torch.tensor([len(params)], device=device)
+    if world > 1:
+        dist.all_reduce(n_files)
+    cap = (DUMP_LIMIT_BYTES // (int(n_files.item()) + 1) - NPY_HEADER_BYTES) // 4  # +1: loss.npy
+    os.makedirs(out_dir, exist_ok=True)
+    if rank == 0 and loss is not None:
+        np.save(os.path.join(out_dir, "loss.npy"), np.asarray(loss, dtype=np.float32))
+    for name, p in params:
+        flat = p.detach().reshape(-1).float().cpu().numpy()
+        if flat.size > cap:
+            flat = flat[np.random.RandomState(0).randint(0, flat.size, cap)]
+        np.save(os.path.join(out_dir, name + ".npy"), flat)
 
 
 def _dump_trace(eng, rank, world, device, N):
