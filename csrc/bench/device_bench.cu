@@ -31,10 +31,10 @@ void ckrc(int rc, const char* what) {
 // attention / memory-bound kernels are slow relative to its GEMMs is mis-ranked by such a proxy.
 std::pair<double, double> device_benchmark(int tokens, int hidden, int intermediate, int iterations,
                                            int warmup, double slowdown, int mode, int seq,
-                                           int heads) {
+                                           int heads, int head_dim) {
   const size_t M = tokens, H = hidden, I = intermediate;
-  const bool full = mode == 0 && seq == 128 && heads > 0 && hidden == heads * 64 &&
-                    tokens % seq == 0;
+  const bool full = mode == 0 && heads > 0 && hidden == heads * head_dim &&
+                    attention_supported(seq, head_dim) && tokens % seq == 0;
   std::vector<void*> allocs;
   auto dmalloc = [&](size_t bytes, int fill) {
     void* p = nullptr;
@@ -127,7 +127,7 @@ std::pair<double, double> device_benchmark(int tokens, int hidden, int intermedi
     } else {
       AttnArgs a;
       a.qkv = qkv; a.ctx = ctx; a.lse = lse; a.B = tokens / seq; a.S = seq; a.heads = heads;
-      a.head_dim = 64;
+      a.head_dim = head_dim;
       ckrc(launch_attention_fwd(a, s), "attention_fwd");
       dense_ln(ctx, hidden, wo, hidden, x, z1, "gemm attn-out (+LN)");
       ck(cudaMemcpyAsync(h1, out, M * H * 2, cudaMemcpyDeviceToDevice, s), "copy");
@@ -170,7 +170,7 @@ std::pair<double, double> device_benchmark(int tokens, int hidden, int intermedi
     {
       AttnArgs a;
       a.qkv = qkv; a.ctx = ctx; a.lse = lse; a.dctx = dctx; a.dqkv = dqkv; a.B = tokens / seq;
-      a.S = seq; a.heads = heads; a.head_dim = 64;
+      a.S = seq; a.heads = heads; a.head_dim = head_dim;
       ckrc(launch_attention_bwd(a, s), "attention_bwd");
     }
     gemm(dqkv, 3 * hidden, true, x, hidden, true, 3 * hidden, hidden, tokens, gw_qkv, hidden,

@@ -9,9 +9,10 @@
 
 namespace sky {
 // returns (total seconds for `iterations` proxy blocks incl. simulated slowdown, free HBM in MiB)
-// mode 0 = full forward + backward block (needs seq == 128, hidden == heads * 64; falls back to
-// mode 1 otherwise), mode 1 = the four forward GEMMs only
+// mode 0 = full forward + backward block (needs hidden == heads * head_dim, an attention shape
+// the kernels support and tokens % seq == 0; falls back to mode 1 otherwise), mode 1 = the four
+// forward GEMMs only
 std::pair<double, double> device_benchmark(int tokens, int hidden, int intermediate, int iterations,
                                            int warmup, double slowdown, int mode = 0,
-                                           int seq = 128, int heads = 16);
+                                           int seq = 128, int heads = 16, int head_dim = 64);
 }  // namespace sky

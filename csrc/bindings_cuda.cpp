@@ -503,7 +503,7 @@ PYBIND11_MODULE(_cuda, m) {
   m.def("device_benchmark", &sky::device_benchmark, py::arg("tokens"), py::arg("hidden"),
         py::arg("intermediate"), py::arg("iterations"), py::arg("warmup"),
         py::arg("slowdown") = 0.0, py::arg("mode") = 0, py::arg("seq") = 128,
-        py::arg("heads") = 16,
+        py::arg("heads") = 16, py::arg("head_dim") = 64,
         "C++ device benchmark loop: times `iterations` transformer blocks (mode 0: the full "
         "forward + backward kernel chain, mode 1: forward GEMMs only) with CUDA events; returns "
         "(seconds_total, free_mem_MiB)");

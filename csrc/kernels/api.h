@@ -129,10 +129,11 @@ int launch_dgelu_mul(const void* g, const void* h, void* y, long long n, cudaStr
 int launch_colsum(const void* x_bf16, int M, int N, int ldx, float* out, cudaStream_t stream);
 
 // ---------------------------------------------------------------------------------------------
-// Attention (head_dim = 64; S = 128 single-tile kernels, any other S % 8 == 0 tiled), tcgen05
+// Attention, tcgen05: any S % 8 == 0 and head_dim % 8 == 0 with 8 <= head_dim <= 128 (S = 128 with
+// head_dim = 64: single-tile kernels; everything else tiled); other shapes return 930
 // ---------------------------------------------------------------------------------------------
 struct AttnArgs {
-  const void* qkv = nullptr;   // bf16 [B*S, 3*H]  (Q | K | V), head h at columns h*64
+  const void* qkv = nullptr;   // bf16 [B*S, 3*H]  (Q | K | V), head h at columns h*head_dim
   const float* mask = nullptr; // fp32 additive [B, S] or null
   void* ctx = nullptr;         // bf16 [B*S, H] (fwd: output, bwd: saved forward output)
   float* lse = nullptr;        // fp32 [B*heads, S] log2-domain log-sum-exp (fwd: out, bwd: in)
@@ -146,7 +147,7 @@ struct AttnArgs {
 };
 int launch_attention_fwd(const AttnArgs& a, cudaStream_t stream);
 int launch_attention_bwd(const AttnArgs& a, cudaStream_t stream);
-// any S with S % 8 == 0 (flash-style tiling over 128-key blocks; backward = dQ kernel + dK/dV kernel)
+// every supported shape (flash-style tiling over 128-key blocks; backward = dQ kernel + dK/dV kernel)
 int launch_attention_fwd_tiled(const AttnArgs& a, cudaStream_t stream);
 int launch_attention_bwd_tiled(const AttnArgs& a, cudaStream_t stream);
 bool attention_supported(int S, int head_dim);

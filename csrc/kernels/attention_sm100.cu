@@ -1,4 +1,5 @@
 // Fused self-attention for BERT geometry (S = 128 keys per sequence, head_dim = 64) on tcgen05.
+// Every other sequence length and head size goes to the tiled kernels (attention_tiled_sm100.cu).
 //
 // One CTA per (batch, head).  With S = 128 a whole score matrix is exactly one 128x128 UMMA tile,
 // so no online-softmax tiling is needed:
@@ -441,8 +442,9 @@ attention_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv,
 
 }  // namespace
 
-// S = 128 runs the single-tile kernels of this file; every other length (and S = 128 when
-// SKY_ATTN_TILED=1, for A/B comparisons) the flash-style tiled kernels of attention_tiled_sm100.cu
+// S = 128 with head_dim = 64 runs the single-tile kernels of this file; every other shape (and
+// S = 128 when SKY_ATTN_TILED=1, for A/B comparisons) the flash-style tiled kernels of
+// attention_tiled_sm100.cu, which also reject (930) what no kernel supports
 static bool force_tiled() {
   static int v = -1;
   if (v < 0) {
@@ -453,8 +455,7 @@ static bool force_tiled() {
 }
 
 int launch_attention_fwd(const AttnArgs& a, cudaStream_t stream) {
-  if (a.head_dim != kD) return 930;
-  if (a.S != kS || force_tiled()) return launch_attention_fwd_tiled(a, stream);
+  if (a.head_dim != kD || a.S != kS || force_tiled()) return launch_attention_fwd_tiled(a, stream);
   if (a.dropout_p > 0.f && a.rng_state == nullptr) return 903;
   const int H = a.heads * kD;
   CUtensorMap tm;
@@ -486,8 +487,7 @@ int launch_attention_fwd(const AttnArgs& a, cudaStream_t stream) {
 }
 
 int launch_attention_bwd(const AttnArgs& a, cudaStream_t stream) {
-  if (a.head_dim != kD) return 930;
-  if (a.S != kS || force_tiled()) return launch_attention_bwd_tiled(a, stream);
+  if (a.head_dim != kD || a.S != kS || force_tiled()) return launch_attention_bwd_tiled(a, stream);
   if (a.dropout_p > 0.f && a.rng_state == nullptr) return 903;
   if (a.lse == nullptr || a.ctx == nullptr || a.dctx == nullptr) return 931;
   const int H = a.heads * kD;

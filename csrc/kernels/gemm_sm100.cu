@@ -1143,6 +1143,23 @@ int make_tmap_bf16_3d(CUtensorMap* tm, const void* ptr, uint64_t inner, uint64_t
   return r == CUDA_SUCCESS ? 0 : 1000 + static_cast<int>(r);
 }
 
+// 4D bf16 tensor map, dims[0] contiguous, ld_elems[i] = stride of dims[i + 1]; box
+// (box_inner, 1, box_third, 1).  The attention kernels view [B * S, sections * D] activations as
+// (D, sections, S, B): a box wider than D then reads zeros past the end of a head's columns.
+int make_tmap_bf16_4d(CUtensorMap* tm, const void* ptr, const uint64_t (&dims)[4],
+                      const uint64_t (&ld_elems)[3], uint32_t box_inner, uint32_t box_third) {
+  PFN_encodeTiled enc = get_encode_fn();
+  if (!enc) return 901;
+  cuuint64_t gdim[4] = {dims[0], dims[1], dims[2], dims[3]};
+  cuuint64_t gstride[3] = {ld_elems[0] * 2, ld_elems[1] * 2, ld_elems[2] * 2};
+  cuuint32_t box[4] = {box_inner, 1, box_third, 1};
+  cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), gdim, gstride,
+                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return r == CUDA_SUCCESS ? 0 : 1000 + static_cast<int>(r);
+}
+
 int gemm_pick_block_n(int M, int N) {
   // 256-wide tiles halve B re-reads and give the best tensor-pipe duty cycle; fall back to 128
   // when that would leave most SMs idle or N is small.

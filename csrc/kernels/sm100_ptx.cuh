@@ -116,6 +116,18 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* t
       : "memory");
 }
 
+// 4D tiled load; the tiled attention kernels for head sizes other than 64 (zero-filled columns
+// past the head size as well as rows past the sequence end).
+__device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* tmap, uint64_t* bar,
+                                            int c0, int c1, int c2, int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, "
+      "%4, %5, %6}], [%2];"
+      ::"r"(smem_u32(smem_dst)),
+      "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+
 // ----------------------------------------------------------------------------------------------
 // tcgen05: TMEM allocation
 // ----------------------------------------------------------------------------------------------

@@ -80,6 +80,7 @@ class DeviceBenchmarker(BaseBenchmarker):
         dev = cfg.get("cuda_device", -1)
         if dev is not None and dev >= 0:
             torch.cuda.set_device(dev)
+        head_dim = int(block_shape.get("head_dim", 64))
         t, free_mib = nat.ext().device_benchmark(
             tokens=block_shape["tokens"], hidden=block_shape["hidden"],
             intermediate=block_shape["intermediate"], iterations=iterations,
@@ -88,7 +89,8 @@ class DeviceBenchmarker(BaseBenchmarker):
             # LayerNorm, reductions); "gemm_only" selects round 1's four forward GEMMs
             mode=1 if block_shape.get("proxy_kernels") == "gemm_only" else 0,
             seq=int(block_shape.get("seq", 128)),
-            heads=int(block_shape.get("heads", max(1, block_shape["hidden"] // 64))))
+            heads=int(block_shape.get("heads", max(1, block_shape["hidden"] // head_dim))),
+            head_dim=head_dim)
         mem_limit = cfg.get("mem_limit", -1)
         return t, (mem_limit if mem_limit and mem_limit > 0 else free_mib - 500)
 

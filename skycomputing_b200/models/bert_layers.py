@@ -332,10 +332,11 @@ class BertSpan:
         if hidden.dim() != 3 or H % 8 != 0:
             return False
         if self.head is not None:
-            # tcgen05 attention: head size 64, any sequence length that is a multiple of 8 (S = 128
-            # single-tile kernels, everything else flash-style tiles of 128 keys)
-            sa = self.head.attention.self
-            if sa.attention_head_size != 64 or hidden.shape[1] <= 0 or hidden.shape[1] % 8 != 0:
+            # tcgen05 attention: head sizes 8..128 in steps of 8, any sequence length that is a
+            # multiple of 8 (S = 128 / head size 64: single-tile kernels, else flash-style tiles)
+            from ..ops.native import attention_supported
+
+            if not attention_supported(hidden.shape[1], self.head.attention.self.attention_head_size):
                 return False
         if self.body is not None and self.body.intermediate.dense_act.act_name not in ("gelu", "bias_gelu"):
             return False

@@ -331,6 +331,13 @@ def colsum_(x: torch.Tensor, out: torch.Tensor) -> None:
     ext().colsum(x=x.data_ptr(), M=M, N=N, ldx=x.stride(0), out=out.data_ptr(), stream=_stream())
 
 
+def attention_supported(S: int, head_dim: int) -> bool:
+    """Shapes the tcgen05 attention kernels run: any sequence length that is a multiple of 8 and
+    any head size that is a multiple of 8 from 8 to 128.  Pure Python (the same rule as the C++
+    ``attention_supported``), so CPU-only callers can ask without loading the extension."""
+    return S > 0 and S % 8 == 0 and head_dim % 8 == 0 and 8 <= head_dim <= 128
+
+
 def attention_fwd(qkv, mask, B: int, S: int, heads: int, *, dropout_p: float = 0.0,
                   rng: Optional[RngState] = None, rng_stream: int = 0):
     _check(qkv, torch.bfloat16, "qkv")

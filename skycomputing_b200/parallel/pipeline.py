@@ -25,6 +25,7 @@ import torch
 import torch.distributed as dist
 
 from ..builder.module_wrapper import ModuleWrapper
+from ..ops.native import attention_supported
 from .engine_base import EngineBase
 
 
@@ -113,7 +114,8 @@ class PipelineEngine(EngineBase):
             in_ok, out_ok = self.stage.fused_boundary_support((self.mb_batch, self.seq, hidden))
             shape_ok = self.seq % 8 == 0 and hidden % 64 == 0 and (self.mb_batch * self.seq) % 128 == 0
             if spans and spans[0].head is not None:
-                shape_ok = shape_ok and spans[0].head.attention.self.attention_head_size == 64
+                shape_ok = shape_ok and attention_supported(
+                    self.seq, spans[0].head.attention.self.attention_head_size)
             in_ok, out_ok = in_ok and shape_ok, out_ok and shape_ok
         if multi:
             flags: List[tuple] = [None] * dist.get_world_size(self.group)  # type: ignore[list-item]

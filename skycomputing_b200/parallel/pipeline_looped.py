@@ -31,6 +31,7 @@ from typing import Callable, List, Optional, Sequence
 import torch
 import torch.distributed as dist
 
+from ..ops.native import attention_supported
 from .comm import TorchDistComm
 from .engine_base import EngineBase
 
@@ -138,7 +139,8 @@ class LoopedPipelineEngine(EngineBase):
                     sp = spans[0]
                     if sp.head is not None:
                         hidden = sp.head.attention.output.dense.weight.shape[0]
-                        ok = ok and sp.head.attention.self.attention_head_size == 64
+                        ok = ok and attention_supported(
+                            self.seq, sp.head.attention.self.attention_head_size)
                 in_ok, out_ok = st.fused_boundary_support((self.mb_batch, self.seq, hidden))
                 ok = ok and (in_ok or k == 0) and (out_ok or k == self.total - 1)
             ok = ok and self.seq % 8 == 0 and hidden > 0 and hidden % 64 == 0 and \

@@ -25,6 +25,8 @@ def main():
     ap.add_argument("--schedule", default="1f1b")
     ap.add_argument("--dropout", type=float, default=0.0)
     ap.add_argument("--tag", default="")
+    # attention heads of the hidden-1024 model: 16 = head size 64 (BERT-large), 8 = head size 128
+    ap.add_argument("--heads", type=int, default=16)
     # > 1: looped pipeline (v chunks per GPU); add SKY_LOOPED_FUSED=1 for its fused ring boundary.
     # The loss trajectory must equal the plain pipeline's (same seeds per GLOBAL layer index).
     ap.add_argument("--virtual-stages", type=int, default=1)
@@ -39,7 +41,7 @@ def main():
     dist.init_process_group("nccl", rank=rank, world_size=world, device_id=dev)
     set_backend("native")
     torch.manual_seed(7)
-    cfg = BertConfig(30522, hidden_size=1024, num_hidden_layers=a.layers, num_attention_heads=16,
+    cfg = BertConfig(30522, hidden_size=1024, num_hidden_layers=a.layers, num_attention_heads=a.heads,
                      intermediate_size=4096, hidden_dropout_prob=a.dropout,
                      attention_probs_dropout_prob=a.dropout)
     enc = [dict(layer_type="BertLayer_Head", config=cfg.__dict__),

@@ -4,7 +4,7 @@
 #   tools/run_sanitizer.sh [memcheck|racecheck|synccheck|initcheck] [suite]
 # suite:  gemm     tcgen05 GEMM incl. the GEMM + LayerNorm cluster kernel
 #         rows     LayerNorm fwd/bwd, column sums, softmax-CE, fused optimizers
-#         attn     attention fwd/bwd
+#         attn     attention fwd/bwd (head size 64 and the other head sizes)
 #         layers   embeddings + block + pooler + classifier through the layer classes (embed_fwd /
 #                  embed_bwd / small_linear kernels) and the flag handshake (peer_copy_signal,
 #                  wait_flags, flag-gated GEMM) on one GPU
@@ -30,7 +30,7 @@ case "$SUITE" in rows|all)
   run rows tests/test_kernels_gpu.py tests/test_optim_gpu.py -k "layernorm_fwd_bwd or colsum or softmax_ce or dropout_mask_consistent or fused_optimizer" ;;
 esac
 case "$SUITE" in attn|all)
-  run attn tests/test_kernels_gpu.py -k "attention" ;;
+  run attn tests/test_kernels_gpu.py tests/test_attention_head_dims_gpu.py -k "attention and not engine and not span and not two_gpu" ;;
 esac
 case "$SUITE" in layers|all)
   run layers tests/test_layers_gpu.py tests/test_kernels_gpu.py -k "embeddings_pooler_classifier or handshake or signals_panels" ;;
